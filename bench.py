@@ -23,6 +23,11 @@ parity    after the timed region rank 0 compares the (merged) result with an ind
           A mismatch fails the run.
 cpu_baseline  the CPU oracle (restatement of the reference's goroutine-per-block path; the Go
           reference cannot be built here) on a bounded sample, all host threads.
+
+--dump-outputs DIR  writes what the last timed step of the bench line returned (MatchedCount, every group's
+          key, Count, Samples and histogram fields, time buckets) as DIR/<name>.npy in float64, at most 64 MB.
+          The tables are generated from fixed seeds, so two builds run with the same arguments can be compared
+          array for array.
 """
 import argparse
 import ctypes as C
@@ -62,7 +67,14 @@ def parse():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--extra", default="auto", help="comma list of other configs to run briefly (auto: c2,c4,c5; none)")
     ap.add_argument("--selfcheck", action="store_true", help="multi-GPU: merged result of 4 small queries vs the oracle first")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step of the bench line as DIR/<name>.npy (float64)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's result (--impl ours)")
+    return a
 
 
 def total_rows_for(workload, world, rows_per_gpu, spec_rows):
@@ -158,6 +170,76 @@ def make_query(spec, synth):
     return Q(s, **kw)
 
 
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much
+
+
+def result_arrays(qs):
+    """The fields of a materialised QuerySpec as float64 arrays.  Rows of `groups_*`: the Cumulative row, then
+    the groups in the result's sorted order; rows of `time_*`: every (time bucket, group), buckets ascending and
+    groups by key.  A key is the CRC-32 of its GroupByKey.  Counts and exact sums of the bench tables stay far
+    below 2^53, so they convert exactly.  A group without a histogram holds NaN."""
+    import zlib
+    import numpy as np
+
+    def padded(seqs):
+        m = np.full((len(seqs), max((len(s) for s in seqs if s is not None), default=0)), np.nan)
+        for i, s in enumerate(seqs):
+            if s is not None:
+                m[i, :len(s)] = s
+        return m
+
+    out = {"scalars": np.array([qs.MatchedCount, qs.NumGroups, qs.BrokenBlocks, qs.SkippedBlocks], np.float64)}
+    tables = {"groups": [(None, r) for r in [qs.Cumulative] + qs.Sorted]}
+    if qs.TimeResults:
+        tables["time"] = [(tb, r) for tb, m in sorted(qs.TimeResults.items()) for _, r in sorted(m.items())]
+        out["time_bucket"] = np.array([tb for tb, _ in tables["time"]], np.float64)
+    for t, rows in tables.items():
+        out[t + "_key_crc32"] = np.array([zlib.crc32(r.GroupByKey.encode()) for _, r in rows], np.float64)
+        out[t + "_count"] = np.array([r.Count for _, r in rows], np.float64)
+        out[t + "_samples"] = np.array([r.Samples for _, r in rows], np.float64)
+        for a in qs.Aggregations:
+            hs = [r.Hists.get(a.Name) for _, r in rows]
+            for field, get in (("count", lambda h: h.TotalCount()), ("sum", lambda h: h.Sum()), ("min", lambda h: h.Min()),
+                               ("max", lambda h: h.Max()), ("avg", lambda h: h.Mean()), ("stddev", lambda h: h.StdDev())):
+                out["%s_%s_%s" % (t, a.Name, field)] = np.array([np.nan if h is None else get(h) for h in hs], np.float64)
+            out["%s_%s_percentiles" % (t, a.Name)] = padded([None if h is None else h.GetPercentiles() for h in hs])
+            out["%s_%s_buckets" % (t, a.Name)] = padded([None if h is None else h.Values for h in hs])
+    return out
+
+
+def sample_rows(arrays, limit=DUMP_BYTES):
+    """Arrays larger than `limit` in all keep a fixed, seeded sample of the rows of each table; `<table>_rows`
+    holds the indices kept.  Every row is at least 24 bytes, so the 8-byte index per row fits in the halved share."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total <= limit:
+        return arrays
+    rng = np.random.default_rng(0)
+    for t in ("groups", "time"):
+        names = [k for k in arrays if k.startswith(t + "_")]
+        if names:
+            n = len(arrays[names[0]])
+            idx = np.sort(rng.choice(n, max(1, int(n * limit / (2 * total))), replace=False))
+            for k in names:
+                arrays[k] = arrays[k][idx]
+            arrays[t + "_rows"] = idx.astype(np.float64)
+    return arrays
+
+
+def dump_outputs(path, table, qs):
+    """--dump-outputs: materialise the result the last timed step kept (qs.result) and write its arrays."""
+    import numpy as np
+    try:
+        qs.materialize = True
+        table._fill(qs, qs.result)
+    finally:
+        table.lib.sg_result_free(qs.result)
+        qs.result = None
+    os.makedirs(path, exist_ok=True)
+    for name, a in sample_rows(result_arrays(qs)).items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def host_info():
     info = {"nproc": os.cpu_count()}
     try:
@@ -243,8 +325,9 @@ class Env:
 CHUNK_LIMIT = 12 << 30  # pinned arena the blocks are generated into and staged from
 
 
-def run_workload(env, workload, rows_per_gpu, steps, warmup, do_e2e, e2e_steps, do_cpu, do_parity):
-    """One config on this job's GPUs.  Returns the JSON line's fields (rank 0) or None (other ranks)."""
+def run_workload(env, workload, rows_per_gpu, steps, warmup, do_e2e, e2e_steps, do_cpu, do_parity, dump_dir=None):
+    """One config on this job's GPUs.  Returns the JSON line's fields (rank 0) or None (other ranks).
+    dump_dir: rank 0 writes the result of the last timed step there (dump_outputs)."""
     from sybil_b200 import _ffi as F
     from sybil_b200 import engine as E
     from sybil_b200 import synth
@@ -303,7 +386,7 @@ def run_workload(env, workload, rows_per_gpu, steps, warmup, do_e2e, e2e_steps, 
 
     prepared = {}
 
-    def one_step(tbl, materialize=False):
+    def one_step(tbl, materialize=False, keep_result=False):
         """One query = one step.  The query is prepared once per table (QuerySpec -> sg_query_begin), as a host
         that repeats a dashboard query would; every step runs the scan, the merge and the result read-back."""
         qs = q.query_spec()
@@ -315,7 +398,7 @@ def run_workload(env, workload, rows_per_gpu, steps, warmup, do_e2e, e2e_steps, 
             for c in spec.cols:
                 (ls.Int if c.col_type == F.SG_COL_INT else ls.Str)(c.name)
             pq = prepared[id(tbl)] = tbl.Prepare(ls, qs)
-        pq.Run(qs, allreduce=world > 1)
+        pq.Run(qs, allreduce=world > 1, keep_result=keep_result)
         return qs
 
     # ---- value: resident inputs -----------------------------------------------------------
@@ -328,13 +411,16 @@ def run_workload(env, workload, rows_per_gpu, steps, warmup, do_e2e, e2e_steps, 
     env.barrier()
     t0 = time.perf_counter()
     kernel_ms, launches = 0.0, 0
-    for _ in range(steps):
-        qs = one_step(table)
+    keep_last = dump_dir is not None and rank == 0
+    for i in range(steps):
+        qs = one_step(table, keep_result=keep_last and i == steps - 1)
         kernel_ms += qs.stats.kernel_ms
         launches += qs.stats.kernel_launches
     env.barrier()
     elapsed = env.max_over_ranks(time.perf_counter() - t0)
     clocks = sampler.finish() if sampler else None
+    if keep_last:
+        dump_outputs(dump_dir, table, qs)
     total_rows = env.sum_over_ranks(float(my_rows))
     ms_per_step = elapsed / steps * 1e3
     value = total_rows / (elapsed / steps)
@@ -482,7 +568,7 @@ def run_ours(args):
         except Exception as e:  # noqa: BLE001
             sc = {"ok": False, "error": repr(e)[:300]}
     line = run_workload(env, args.workload, args.rows, args.steps, args.warmup, not args.no_e2e, args.e2e_steps,
-                        not args.no_cpu, not args.no_parity)
+                        not args.no_cpu, not args.no_parity, args.dump_outputs)
     extras = []
     names = [] if args.extra == "none" else (["c2", "c4", "c5"] if args.extra == "auto" else args.extra.split(","))
     if args.rows and args.extra == "auto":

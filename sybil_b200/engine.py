@@ -530,9 +530,10 @@ class PreparedQuery:
             self.Close()
             raise
 
-    def Run(self, qs, allreduce=False):
+    def Run(self, qs, allreduce=False, keep_result=False):
         """One pass of the hot path; fills qs like LoadAndQueryRecords.  The result object is freed before
-        the call returns (the Python mirror copies what it exposes)."""
+        the call returns (the Python mirror copies what it exposes), unless keep_result: then it stays alive
+        as qs.result (Table._fill materialises it later) and the caller frees it with sg_result_free."""
         t = self.table
         lib, ctx = t.lib, t.ctx
         ctx.check(lib.sg_query_run(self.q))
@@ -545,7 +546,12 @@ class PreparedQuery:
         qs.stats = st
         try:
             t._fill(qs, rp)
-        finally:
+        except BaseException:
+            lib.sg_result_free(rp)
+            raise
+        if keep_result:
+            qs.result = rp
+        else:
             lib.sg_result_free(rp)
         return qs.MatchedCount
 
